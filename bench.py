@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps 2 --warmup 1       # the unmodified reference (oracle/_ref archive) on host cores
+    python bench.py --steps 20 --warmup 3 --dump-outputs /tmp/out   # + the last timed step's outputs as /tmp/out/*.npy
 
 Workload (BASELINE.json configs[1]): v2_ctc, batch 64 x 10 s synthetic 16 kHz audio per GPU (weak scaling:
 every rank runs its own 64 utterances, hypotheses all-gathered to every rank over NCCL when N > 1), seeded
@@ -35,6 +36,7 @@ MODEL = "v2_ctc"
 BATCH = 64
 SECONDS = 10.0
 N_ROT = 4  # rotating input buffers: 4 x 41 MB = 164 MB > 126 MB L2
+DUMP_LIMIT = 64_000_000  # bytes of .npy data --dump-outputs may write
 
 
 def flops_per_utterance(n_samples: int) -> dict:
@@ -179,6 +181,31 @@ def cpu_reference(steps: int, warmup: int, batch: int = 4, reps: int = 3, second
             "rtfx": batch * reps * seconds / sec, "sec_per_step": sec}
 
 
+def dump_outputs(out_dir: Path, enc, enc_len, ids, frames, counts) -> None:
+    """What one step of the timed path returned (encoder output and lengths, CTC hypotheses), written as float32 / float64
+    .npy files so that two builds can be compared output for output on the same seeded inputs.  Hypothesis slots past an
+    utterance's count hold -1 (the kernels leave them unwritten).  If the encoder output [B, T', d] would not fit in
+    DUMP_LIMIT, a fixed seeded sample of utterances is written; enc_utterances.npy lists which."""
+    import numpy as np
+    import torch
+
+    out_dir.mkdir(parents=True, exist_ok=True)
+    counts = counts.cpu().long()
+    unwritten = torch.arange(ids.shape[1])[None, :] >= counts[:, None]
+    arrays = {"enc_len": enc_len.cpu().double(), "counts": counts.double(),
+              "ids": ids.cpu().long().masked_fill(unwritten, -1).double(),
+              "frames": frames.cpu().long().masked_fill(unwritten, -1).double()}
+    B = enc.shape[0]
+    room = (DUMP_LIMIT - 8 * sum(a.numel() for a in arrays.values()) - 8 * B - 4096) // (4 * enc[0].numel())  # 4 KB: headers
+    keep = torch.arange(B)
+    if room < B:
+        keep = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:room].sort().values
+    arrays["enc_utterances"] = keep.double()
+    arrays["enc"] = enc[keep.to(enc.device)].float().cpu()
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a.numpy())
+
+
 def c4_strong_scaling(dev, rank: int, world: int, steps: int = 3, total: int = 256, chunk: int = 32, seconds: float = 10.0):
     """BASELINE.json configs[3]: v3_e2e_rnnt, 256 x 10 s in total, sharded across the N GPUs of the job (STRONG scaling:
     the work is fixed, 256 / N utterances per rank, run in device batches of 32 = the per-GPU batch at N = 8), encoder +
@@ -247,7 +274,13 @@ def main():
     ap.add_argument("--batch", type=int, default=BATCH)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c4", action="store_true", help="skip the strong-scaling leg (BASELINE configs[3])")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 path")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -265,7 +298,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return 0
-        steps = max(1, min(args.steps, 5))
+        steps = args.steps
         res = cpu_reference(steps, max(1, min(args.warmup, 1)))
         line = {"impl": "reference", "metric": "utterances/sec (10 s audio, v2_ctc)", "value": res["value"], "unit": "utt/s",
                 "n_gpus": args.gpus, "steps": steps, "warmup": 1, "ms_per_step": res["sec_per_step"] * 1e3, "higher_is_better": True,
@@ -311,8 +344,8 @@ def main():
         enc, enc_len = eng.encode(mel, mel_len)
         ids, frames, counts = eng.greedy(enc, enc_len, packed)
         if hyp_gather is not None and collective:
-            return ids, frames, counts, hyp_gather.all_gather(packed)
-        return ids, frames, counts, None
+            return ids, frames, counts, hyp_gather.all_gather(packed), enc, enc_len
+        return ids, frames, counts, None, enc, enc_len
 
     # ---- warm-up eagerly, then capture the whole step in one CUDA graph (kills ~250 launch gaps)
     side = torch.cuda.Stream(device=dev)
@@ -326,7 +359,7 @@ def main():
     side.synchronize()
     graph = torch.cuda.CUDAGraph()
     with torch.cuda.graph(graph, stream=side):
-        g_ids, g_frames, g_counts, g_all = device_step(static_in)
+        g_ids, g_frames, g_counts, g_all, g_enc, g_enc_len = device_step(static_in)
 
     def graph_step(i):
         static_in.copy_(wavs[i % N_ROT], non_blocking=True)  # device->device refill of the static input (41 MB)
@@ -359,6 +392,9 @@ def main():
     ms_total = float(t.item())
     ms_per_step = ms_total / args.steps
     value = world * B * args.steps / (ms_total / 1e3)
+    if args.dump_outputs is not None and rank == 0:
+        # before any later leg: the eager runs below write into the same hypothesis buffer
+        dump_outputs(args.dump_outputs, g_enc, g_enc_len, g_ids, g_frames, g_counts)
 
     # ---- end to end through the public API from pinned host memory
     host_wavs = [w.cpu().pin_memory() for w in wavs]

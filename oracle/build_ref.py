@@ -30,7 +30,11 @@ ARCHIVE = OUT / "gigaam_ref.zip"
 
 def build_ref(quiet: bool = False):
     src = REF / "gigaam"
-    if not src.is_dir():
+    try:
+        present = src.is_dir()
+    except OSError:          # not readable by this user: the same as absent
+        present = False
+    if not present:
         if not quiet:
             print(f"{src} not present: keeping whatever oracle/_ref already holds")
         return ARCHIVE if ARCHIVE.is_file() else None

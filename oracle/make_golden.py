@@ -1,7 +1,8 @@
-"""Generate tests/golden/*.npz from the REAL reference (run in the build container, where /root/reference
-exists) and pin oracle/gigaam_oracle.py against it.
+"""Generate the fixtures under tests/golden/ from the REAL reference (run where the reference package is readable,
+oracle/ref_loader.py) and pin oracle/gigaam_oracle.py against it.
 
     python oracle/make_golden.py            # writes fixtures, asserts oracle == reference
+    python oracle/make_golden.py ragged_v1_ctc word_grouping   # only the named cases
 
 The reference cannot be imported as a package offline (hydra / omegaconf / soundfile are absent,
 gigaam/model.py:3-4, gigaam/utils.py:9), so those three are stubbed and its hot-path classes are built
@@ -84,6 +85,68 @@ def run_case(model_name: str, batch: int, seconds: float, ragged: bool, out_name
     return report
 
 
+RAGGED_SECONDS = [4.0, 0.06, 1.3, 3.1, 0.5, 4.0]   # one 4 s buffer, utterances from full length down to two encoder frames
+RAGGED_CHANNELS = 32                               # encoder channels kept per valid frame (a seeded sample of the 768)
+
+
+def run_ragged_case(model_name: str):
+    """The reference's encoder lengths and output on a strongly ragged batch (3 layers deep).  Every valid frame is kept,
+    for a fixed sample of the channels, so that the file stays small while a masking or length error still shows."""
+    from gigaam_b200 import synthetic
+    from oracle import gigaam_oracle as orc
+
+    ck = synthetic.synthetic_checkpoint(model_name, seed=0, n_layers=3)
+    root, _ = build_reference(ck["cfg"], ck["state_dict"])
+    wav, _ = synthetic.synthetic_audio(len(RAGGED_SECONDS), 4.0, seed=4321)
+    wav_len = torch.tensor([int(s * 16000) for s in RAGGED_SECONDS])
+    for b, n in enumerate(wav_len.tolist()):
+        wav[b, n:] = 0.0
+    with torch.inference_mode():
+        mel, mel_len = root.preprocessor(wav, wav_len)
+        enc, enc_len = root.encoder(mel, mel_len)
+        enc_o, enc_len_o = orc.model_forward(wav, wav_len, ck["state_dict"], ck["cfg"])
+    assert torch.equal(enc_len.long(), enc_len_o.long()), (enc_len, enc_len_o)
+    channels = np.sort(np.random.default_rng(0).choice(enc.shape[1], RAGGED_CHANNELS, replace=False))
+    ch = torch.from_numpy(channels)
+    enc_valid = torch.cat([enc[b][ch, :n].t() for b, n in enumerate(enc_len.tolist())])     # [sum(enc_len), channels]
+    out = ROOT / "tests" / "golden" / f"ragged_{model_name}_l3.npz"
+    np.savez_compressed(out, wav_len=wav_len.numpy(), enc_len=enc_len.numpy(), channels=channels,
+                        enc_valid=enc_valid.numpy().astype(np.float32))
+    print(out.name, enc_len.tolist(), f"{out.stat().st_size / 1024:.0f} KiB")
+
+
+WORD_PIECES = ["▁", "▁ab", "cd", "▁e", "f", "▁ ", "g", "▁hij", "k", " ", "\t", "lm"]
+
+
+def run_word_grouping_case():
+    """The reference's frames_to_words on 300 random hypotheses over a small SentencePiece-like vocabulary: leading,
+    trailing and repeated delimiters, bare U+2581 pieces, whitespace-only pieces, empty hypotheses."""
+    import json
+    import random
+    from oracle.ref_loader import import_reference
+    import_reference()
+    import gigaam.timestamps_utils as ref_ts
+
+    class Pieces:
+        def __len__(self):
+            return len(WORD_PIECES)
+
+        def id_to_str(self, i):
+            return WORD_PIECES[i]
+
+    rng = random.Random(0)
+    cases = []
+    for _ in range(300):
+        n = rng.randint(0, 40)
+        ids = [rng.randrange(len(WORD_PIECES)) for _ in range(n)]
+        frames = sorted(rng.randrange(300) for _ in range(n))
+        words = [[w.text, w.start, w.end] for w in ref_ts.frames_to_words(Pieces(), ids, frames, 0.04)]
+        cases.append({"ids": ids, "frames": frames, "words": words})
+    out = ROOT / "tests" / "golden" / "word_grouping.json"
+    out.write_text(json.dumps({"pieces": WORD_PIECES, "frame_shift": 0.04, "cases": cases}, separators=(",", ":")) + "\n")
+    print(out.name, f"{out.stat().st_size / 1024:.0f} KiB")
+
+
 if __name__ == "__main__":
     torch.set_num_threads(os.cpu_count() or 8)
     cases = {
@@ -94,5 +157,10 @@ if __name__ == "__main__":
         # v1 shape: the rel_pos attention branch (encoder.py:191-228, 307-334); 6 s so that T' = 151 spans two key blocks
         "v1_ctc": dict(batch=2, seconds=6.0, ragged=True, out_name="v1_ctc_b2_6s.npz"),
     }
-    for name in (sys.argv[1:] or list(cases)):
-        run_case(name, **cases[name])
+    extra = {f"ragged_{m}": (lambda m=m: run_ragged_case(m)) for m in ("v2_ctc", "v3_e2e_rnnt", "v1_ctc")}
+    extra["word_grouping"] = run_word_grouping_case
+    for name in (sys.argv[1:] or list(cases) + list(extra)):
+        if name in extra:
+            extra[name]()
+        else:
+            run_case(name, **cases[name])

@@ -26,8 +26,11 @@ def reference_root() -> str | None:
     """sys.path entry that provides the reference's `gigaam` package, or None."""
     if os.environ.get("GIGAAM_REFERENCE_ARCHIVE_ONLY", "0") != "1":
         for cand in (os.environ.get("GIGAAM_REFERENCE"), "/root/reference"):
-            if cand and (Path(cand) / "gigaam" / "encoder.py").is_file():
-                return cand
+            try:
+                if cand and (Path(cand) / "gigaam" / "encoder.py").is_file():
+                    return cand
+            except OSError:  # not readable by this user: try the next candidate
+                pass
     return str(ARCHIVE) if ARCHIVE.is_file() else None
 
 

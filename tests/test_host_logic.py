@@ -345,26 +345,19 @@ class _Pieces:
         return self.pieces[i]
 
 
-def test_word_grouping_restatement_and_flag_table_match_the_reference():
-    """gigaam_b200.timestamps_utils.frames_to_words against the reference's own function (imported from /root/reference or
-    the compiled oracle/_ref archive) on random hypotheses, and the per-token flag table the device kernel consumes."""
-    import random
+def test_word_grouping_restatement_and_flag_table_match_the_reference(golden_dir):
+    """gigaam_b200.timestamps_utils.frames_to_words against what the reference's own function returned on 300 random
+    hypotheses (tests/golden/word_grouping.json, oracle/make_golden.py), and the per-token flag table the device kernel
+    consumes."""
+    import json
     from gigaam_b200.timestamps_utils import frames_to_words, token_flag_table
     tok = _Pieces(["▁", "▁ab", "cd", "▁e", "f", "▁ ", "g", "▁hij", "k", " ", "\t", "lm"])
     assert token_flag_table(tok).tolist() == [2 | 4, 2, 0, 2, 0, 2 | 4, 0, 2, 0, 1, 4, 0]
-    try:
-        from oracle.ref_loader import import_reference
-        import_reference()
-        import gigaam.timestamps_utils as ref_ts
-    except ImportError:
-        pytest.skip("reference not importable here (neither /root/reference nor oracle/_ref)")
-    rng = random.Random(0)
-    for _ in range(300):
-        n = rng.randint(0, 40)
-        ids = [rng.randrange(len(tok)) for _ in range(n)]
-        frames = sorted(rng.randrange(300) for _ in range(n))
-        want = [(w.text, w.start, w.end) for w in ref_ts.frames_to_words(tok, ids, frames, 0.04)]
-        assert [(w.text, w.start, w.end) for w in frames_to_words(tok, ids, frames, 0.04)] == want
+    g = json.loads((golden_dir / "word_grouping.json").read_text())
+    assert g["pieces"] == tok.pieces and len(g["cases"]) == 300
+    for case in g["cases"]:
+        got = [[w.text, w.start, w.end] for w in frames_to_words(tok, case["ids"], case["frames"], g["frame_shift"])]
+        assert got == case["words"], case
 
 
 def test_known_answer_transcripts_when_real_checkpoints_are_present():
